@@ -535,6 +535,24 @@ def config4_block(args, dev, rank, world, noise=0):
             "sequential_loop_s_rank0": seq_s}
 
 
+DUMP_IMAGES = 6  # decoded images written in full by --dump-outputs (6 x 832x624x4 float32 = 50 MB)
+
+
+def dump_outputs(where, out):
+    """--dump-outputs (rank 0): what the last timed step left in the monitors' output images, as .npy files (under
+    64 MB in all): `out` = DUMP_IMAGES whole images (n, H, W, BGRA; float32) of monitors drawn with a fixed seed,
+    `out_index` = which monitors they are (float32), `out_sums` = the per-channel sum of every monitor's image (B, 4;
+    float64, exact)."""
+    import numpy as np
+    import torch
+    os.makedirs(where, exist_ok=True)
+    pick = np.sort(np.random.default_rng(0).choice(out.shape[0], size=min(DUMP_IMAGES, out.shape[0]), replace=False))
+    idx = torch.from_numpy(pick).to(out.device)
+    np.save(os.path.join(where, "out.npy"), out.index_select(0, idx).float().cpu().numpy())
+    np.save(os.path.join(where, "out_index.npy"), pick.astype(np.float32))
+    np.save(os.path.join(where, "out_sums.npy"), out.sum(dim=(1, 2), dtype=torch.float64).cpu().numpy())
+
+
 def run_product(args):
     import numpy as np  # noqa: F401
     import torch
@@ -625,6 +643,8 @@ def run_product(args):
     barrier()
     ms = ev0.elapsed_time(ev1)
     clocks = sampler.finish()
+    if args.dump_outputs and rank == 0:  # the last timed step's images, before the passes below overwrite them
+        dump_outputs(args.dump_outputs, out)
     launches = batch.launches - launches0
     took_lines2 = batch.lines2_launches - lines2_0
     batch.set_option("timing", 1)
@@ -903,6 +923,8 @@ def main():
     ap.add_argument("--config4-segments", type=int, default=0, help="time-parallel segments per rank (0: about 8 frames per segment)")
     ap.add_argument("--set", action="append", default=[], help="library option name=value (A/B testing)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the images the last timed step computed to DIR/*.npy (a seeded sample; see dump_outputs)")
     ap.add_argument("--no-allgather", action="store_true", help="N > 1: skip the all_gather / gather_to_root blocks")
     ap.add_argument("--no-numa", action="store_true", help="do not bind the process to the GPU's NUMA node")
     ap.add_argument("--variant", default="ntsc", choices=["ntsc", "ntsc_conv", "ntsc_conv6", "ntsc_conv5", "ntsc_conv4", "nes", "nes_p0", "nes_p1", "snes", "nesrgb", "nesrgb_p0", "nesrgb_p1", "vhs", "template", "pv1k", "ntsc_bloom"],

@@ -17,6 +17,16 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
 
 
+def pytest_runtest_setup(item):
+    import support
+    support.begin_test(item)  # the reference results a test compares with are counted per run of it
+
+
+def pytest_runtest_teardown(item, nextitem):
+    import support
+    support.end_test()
+
+
 def _cuda_ok():
     try:
         import torch

@@ -8,8 +8,15 @@
 
 All of them expose: set(**knobs), modulate(img, **settings), demodulate(noise) and the
 state arrays analog / inp / out / ccf / hsync / vsync / rn.
+
+Where the compiled reference is absent (it can only be built next to the reference's
+sources), RefEngine and ref_result() replay what the reference produced in the same test,
+recorded under tests/golden/reference/ (see ref_result).
 """
+import atexit
 import ctypes as C
+import hashlib
+import json
 import os
 
 import numpy as np
@@ -33,6 +40,84 @@ def ref_path(variant):
 
 def have_ref(variant="ntsc"):
     return os.path.exists(ref_path(variant))
+
+
+# ----------------------------------------------------------------------------------
+# recorded reference results
+# ----------------------------------------------------------------------------------
+
+REF_GOLDEN_DIR = os.path.join(ROOT, "tests", "golden", "reference")
+# a directory to write the reference results of this run into (tests/golden/reference/ to refresh the goldens)
+REF_RECORD_DIR = os.environ.get("CRT_REF_RECORD")
+
+_recorded = {}   # module -> {test: [result, ...]} written at exit when REF_RECORD_DIR is set
+_golden = {}     # module -> {test: [result, ...]} loaded from REF_GOLDEN_DIR
+_run = None      # the running test: [module, test, position of its next result, results so far]
+
+
+def begin_test(item):
+    """Start the reference results of one run of a pytest item (tests/conftest.py calls it before every test).  They
+    are keyed by the file and function that define the test, plus its parameters: tests/test_simt_kernels.py runs the
+    GPU tests again under other names and replays the same recordings."""
+    global _run
+    fn = getattr(item, "function", None)
+    if fn is None:
+        _run = None
+        return
+    callspec = getattr(item, "callspec", None)
+    test = fn.__name__ + ("[%s]" % callspec.id if callspec is not None else "")
+    _run = [os.path.basename(fn.__code__.co_filename), test, 0, []]
+
+
+def end_test():
+    """Close the running test's results; a recording run keeps the first run of every key."""
+    global _run
+    if _run is not None and REF_RECORD_DIR and _run[3]:
+        _recorded.setdefault(_run[0], {}).setdefault(_run[1], _run[3])
+    _run = None
+
+
+def digest(a):
+    """short content digest of an array (bytes and shape)"""
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(repr(a.shape).encode() + a.tobytes()).hexdigest()[:16]
+
+
+def ref_result(compute, live):
+    """One result of the compiled reference in the running test, in call order.
+
+    live: the compiled reference this result comes from exists -- compute() is called and its value (anything JSON
+    can hold; digest() for arrays) returned, and recorded when CRT_REF_RECORD names a directory.  Otherwise the value
+    recorded at the same position of the same test under tests/golden/reference/<test module>.json is returned."""
+    assert _run is not None, "ref_result() is called from inside a test function (begin_test() starts its results)"
+    module, test, pos, results = _run
+    _run[2] = pos + 1
+    if live:
+        value = json.loads(json.dumps(compute()))
+        results.append(value)
+        return value
+    if module not in _golden:
+        path = os.path.join(REF_GOLDEN_DIR, module[:-3] + ".json")
+        _golden[module] = json.load(open(path)) if os.path.exists(path) else {}
+    seq = _golden[module].get(test)
+    assert seq is not None and pos < len(seq), (
+        "no recorded reference result %d for %s::%s in tests/golden/reference/ (record it where oracle/_ref is built: "
+        "CRT_REF_RECORD=tests/golden/reference pytest ...)" % (pos, module, test))
+    return seq[pos]
+
+
+@atexit.register
+def _write_recorded():
+    if not (REF_RECORD_DIR and _recorded):
+        return
+    os.makedirs(REF_RECORD_DIR, exist_ok=True)
+    for module, tests in _recorded.items():
+        path = os.path.join(REF_RECORD_DIR, module[:-3] + ".json")
+        old = json.load(open(path)) if os.path.exists(path) else {}
+        old.update(tests)
+        with open(path, "w") as f:  # one test per line
+            f.write("{\n%s\n}\n" % ",\n".join("%s:%s" % (json.dumps(t), json.dumps(old[t], separators=(",", ":")))
+                                               for t in sorted(old)))
 
 
 # ----------------------------------------------------------------------------------
@@ -175,12 +260,62 @@ class CEngine:
                     hsync=self.hsync, vsync=self.vsync, rn=self.rn)
 
 
+class RefState(dict):
+    """A state of the reference; `replayed`: it holds no arrays, assert_same_state compares with the recorded digest."""
+    replayed = False
+
+
+STATE_KEYS = ("hsync", "vsync", "rn", "ccf", "analog", "inp", "out")
+
+
+def state_digest(st):
+    return [int(st["hsync"]), int(st["vsync"]), int(st["rn"]), digest(np.asarray(st["ccf"], dtype=np.int64)),
+            digest(st["analog"]), digest(st["inp"]), digest(st["out"])]
+
+
 class RefEngine(CEngine):
     def __init__(self, variant, outw, outh, fmt=layout.PIX_BGRA, out=None, seed=None):
         super().__init__(ref_path(variant), variant, outw, outh, fmt, out)
         self.lib.ref_srand.argtypes = [C.c_uint]
         if seed is not None:
             self.lib.ref_srand(seed)
+
+    def state(self):
+        return RefState(super().state())
+
+
+class ReplayedRefEngine:
+    """Stands in for RefEngine where oracle/_ref is not built: takes the same calls and does nothing; its states are
+    the ones RefEngine recorded at the same point of the same test (see ref_result)."""
+
+    def __init__(self, variant, outw, outh, fmt=layout.PIX_BGRA, out=None, seed=None):
+        self.out = out if out is not None else np.zeros((outh, outw, max(1, layout.bpp4fmt(fmt))), dtype=np.uint8)
+
+    def set(self, **kw):
+        return self
+
+    def resize(self, outw, outh, fmt, out):
+        self.out = out
+
+    def reset(self):
+        pass
+
+    def modulate(self, img, **kw):
+        pass
+
+    def demodulate(self, noise=0):
+        pass
+
+    def state(self):
+        st = RefState(out=self.out.copy())  # (tests may mask rows of it before comparing)
+        st.replayed = True
+        return st
+
+
+def ref_engine(variant, outw, outh, fmt=layout.PIX_BGRA, out=None, seed=None):
+    """The compiled reference where oracle/_ref has it, else its recorded states."""
+    cls = RefEngine if have_ref(variant) else ReplayedRefEngine
+    return cls(variant, outw, outh, fmt, out, seed)
 
 
 class _OSys(C.Structure):
@@ -392,7 +527,16 @@ class OracleEngine:
 
 
 def assert_same_state(a, b, what=""):
-    """Bit-exact comparison of two engine states with a useful first-mismatch report."""
+    """Bit-exact comparison of two engine states with a useful first-mismatch report.  A state of the reference is
+    also recorded (or, replayed, compared through its recorded digest: see ref_result)."""
+    for ours, ref in ((a, b), (b, a)):
+        if isinstance(ref, RefState):
+            want = ref_result(lambda: state_digest(ref), live=not ref.replayed)
+            if ref.replayed:
+                bad = [k for k, x, y in zip(STATE_KEYS, state_digest(ours), want) if x != y]
+                assert not bad, "%s: %s differ from the reference's recorded state" % (what, ", ".join(bad))
+                return
+            break
     for key in ("hsync", "vsync", "rn"):
         assert a[key] == b[key], "%s %s: %r != %r" % (what, key, a[key], b[key])
     assert np.array_equal(a["ccf"], b["ccf"]), "%s ccf: %r != %r" % (what, a["ccf"], b["ccf"])

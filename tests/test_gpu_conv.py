@@ -1,6 +1,7 @@
 """GPU parity of the USE_CONVOLUTION decoder variant (SURVEY 8a row a11: crt_core.c:85-147, the 7-tap FIR
-eqf): libcrt_b200_ntsc_conv.so against the oracle's FIR line pass and, when oracle/_ref travelled, against
-the reference compiled with USE_CONVOLUTION 1 -- bit for bit, through the drop-in C-ABI and the batch one."""
+eqf): libcrt_b200_ntsc_conv.so against the oracle's FIR line pass and the reference compiled with USE_CONVOLUTION 1
+(oracle/_ref, else its states recorded under tests/golden/reference/) -- bit for bit, through the drop-in C-ABI and the
+batch one."""
 import numpy as np
 import pytest
 
@@ -14,7 +15,7 @@ V = "ntsc_conv"
 def trio(outw, outh, fmt=layout.PIX_BGRA):
     gpu = S.ProductEngine(V, outw, outh, fmt)
     ora = S.OracleEngine(V, outw, outh, fmt)
-    ref = S.RefEngine(V, outw, outh, fmt, seed=1) if S.have_ref(V) else None
+    ref = S.ref_engine(V, outw, outh, fmt, seed=1)
     return gpu, ora, ref
 
 
@@ -26,8 +27,7 @@ def run_all(engines, fn):
 
 def check(gpu, ora, ref, what):
     S.assert_same_state(gpu.state(), ora.state(), what + " [gpu vs oracle]")
-    if ref is not None:
-        S.assert_same_state(gpu.state(), ref.state(), what + " [gpu vs reference]")
+    S.assert_same_state(gpu.state(), ref.state(), what + " [gpu vs reference]")
 
 
 @pytest.mark.parametrize("progressive", [True, False])
@@ -109,7 +109,7 @@ def test_conv_other_kernels(variant):
                                                (100, 80, layout.PIX_ARGB, 1, 0)):
         gpu = S.ProductEngine(variant, outw, outh, fmt)
         ora = S.OracleEngine(variant, outw, outh, fmt)
-        ref = S.RefEngine(variant, outw, outh, fmt, seed=1) if S.have_ref(variant) else None
+        ref = S.ref_engine(variant, outw, outh, fmt, seed=1)
         run_all((gpu, ora, ref), lambda e: e.set(blend=blend, scanlines=scanlines, hue=-20, brightness=11, saturation=13))
         for it in range(4):
             run_all((gpu, ora, ref), lambda e: e.modulate(img, format=layout.PIX_BGRA, as_color=1, field=it & 1,

@@ -1,5 +1,5 @@
-"""GPU parity: the CUDA product library against the oracle (and the compiled reference when
-oracle/_ref travelled with the snapshot), bit for bit, through the C-ABI.
+"""GPU parity: the CUDA product library against the oracle and the reference (compiled in oracle/_ref, else its
+states recorded under tests/golden/reference/), bit for bit, through the C-ABI.
 
 Two layers:
   * drop-in: the reference's own interface (crt_init / crt_modulate / crt_demodulate on host
@@ -19,7 +19,7 @@ pytestmark = pytest.mark.gpu
 def trio(variant, outw, outh, fmt=layout.PIX_BGRA):
     gpu = S.ProductEngine(variant, outw, outh, fmt)
     ora = S.OracleEngine(variant, outw, outh, fmt)
-    ref = S.RefEngine(variant, outw, outh, fmt, seed=1) if S.have_ref(variant) else None
+    ref = S.ref_engine(variant, outw, outh, fmt, seed=1)
     return gpu, ora, ref
 
 
@@ -31,8 +31,7 @@ def run_all(engines, fn):
 
 def check(gpu, ora, ref, what):
     S.assert_same_state(gpu.state(), ora.state(), what + " [gpu vs oracle]")
-    if ref is not None:
-        S.assert_same_state(gpu.state(), ref.state(), what + " [gpu vs reference]")
+    S.assert_same_state(gpu.state(), ref.state(), what + " [gpu vs reference]")
 
 
 @pytest.mark.parametrize("progressive", [True, False])
@@ -99,6 +98,8 @@ def test_burst_lock_from_poked_accumulators(variant):
     vals = [9000000, -9000000, 16000000, -1, -16000000]
 
     def poke(e):
+        if isinstance(e, S.ReplayedRefEngine):  # (nothing to poke: its states are recorded)
+            return
         tab = e.crt.ccf if hasattr(e, "crt") else e.mon.ccf
         for r in range(e.spec.vper):
             for x in range(e.spec.cc_samples):
@@ -144,6 +145,8 @@ def test_poked_signal_extremes(variant):
     vals = rng.choice(np.array([-128, -128, -127, 127, 126, -126, 0], dtype=np.int8), size=pos.size)
 
     def poke(e):
+        if isinstance(e, S.ReplayedRefEngine):
+            return
         if hasattr(e, "crt"):
             buf = np.frombuffer(e.crt, dtype=np.int8, count=n, offset=0)  # analog[] leads the struct (crt_core.h:74-92)
         else:
@@ -272,10 +275,9 @@ def test_dropin_nes(variant):
 @pytest.mark.parametrize("color", [1, 0])
 def test_dropin_vhs(color):
     """config 5: VHS 832x624 noise 24; the drop-in draws from libc rand() like the reference, so the
-    comparison is against the compiled reference with the same srand (needs oracle/_ref)."""
+    comparison is against the oracle's replica of glibc's rand() with the same seed (pinned to the reference by
+    tests/test_oracle_vs_ref.py::test_rand_replica_matches_glibc)."""
     import ctypes as C
-    if not S.have_ref("vhs"):
-        pytest.skip("oracle/_ref not present")
     img = S.bars_image(832, 624)
     libc = C.CDLL(None)
     gpu = S.ProductEngine("vhs", 832, 624)

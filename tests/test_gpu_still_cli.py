@@ -1,6 +1,7 @@
 """tools/crtx_still.c, the batch counterpart of the reference's command-line driver: for every (in, out) pair the file
 it writes must be byte-identical to what the all-reference build of crt_main.c (oracle/_ref/cli_ref_ntsc) writes for
-that pair alone -- PPM and BMP, in and out, every flag of the command line, several images in one run."""
+that pair alone -- PPM and BMP, in and out, every flag of the command line, several images in one run.  Where that build
+is absent, the reference's files are known by the length and digest recorded under tests/golden/reference/."""
 import os
 import struct
 import subprocess
@@ -32,7 +33,7 @@ def write_bmp(path, bgra, bits):
         f.write(head + rows)
 
 
-@pytest.mark.skipif(not (os.path.exists(REF_CLI) and os.path.exists(STILL)), reason="driver binaries not built")
+@pytest.mark.skipif(not os.path.exists(STILL), reason="driver not built")
 @pytest.mark.parametrize("flags,outw,outh,noise,hue", [("-o", 832, 624, 0, 0), ("-op", 640, 480, 12, 30), ("-omf", 333, 250, 24, 0),
                                                        ("-opr", 832, 624, 0, 90), ("-opa", 320, 240, 0, 0)])
 def test_batch_still_driver_is_byte_identical_to_the_reference_cli(tmp_path, flags, outw, outh, noise, hue):
@@ -60,13 +61,17 @@ def test_batch_still_driver_is_byte_identical_to_the_reference_cli(tmp_path, fla
                          stdout=subprocess.PIPE, stderr=subprocess.PIPE, timeout=600)
     assert res.returncode == 0, res.stderr.decode() + res.stdout.decode()
     for i, o in inputs:
-        want = str(tmp_path / ("ref_" + o))
-        subprocess.run([REF_CLI, flags if "o" in flags else flags + "o", str(outw), str(outh), str(noise), str(hue), i, want],
-                       cwd=str(tmp_path), check=True, stdout=subprocess.DEVNULL, timeout=300)
+        def ref_file():
+            want = str(tmp_path / ("ref_" + o))
+            subprocess.run([REF_CLI, flags if "o" in flags else flags + "o", str(outw), str(outh), str(noise), str(hue), i, want],
+                           cwd=str(tmp_path), check=True, stdout=subprocess.DEVNULL, timeout=300)
+            ref = open(want, "rb").read()
+            return [len(ref), S.digest(np.frombuffer(ref, dtype=np.uint8))]
         got = open(tmp_path / o, "rb").read()
-        ref = open(want, "rb").read()
-        assert len(ref) > 1000
-        assert got == ref, "%s -> %s differs from the reference CLI's file (flags %s)" % (i, o, flags)
+        ref_len, ref_digest = S.ref_result(ref_file, os.path.exists(REF_CLI))
+        assert ref_len > 1000
+        assert [len(got), S.digest(np.frombuffer(got, dtype=np.uint8))] == [ref_len, ref_digest], (
+            "%s -> %s differs from the reference CLI's file (flags %s)" % (i, o, flags))
 
 
 def test_usage_errors():

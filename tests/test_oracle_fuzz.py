@@ -1,5 +1,5 @@
 """The seeded random sweep of tests/test_gpu_fuzz.py, run on the CPU between the oracle and the COMPILED
-REFERENCE (oracle/_ref): it widens the pinning of the oracle beyond the hand-picked cases and proves that every
+REFERENCE (oracle/_ref, else its states recorded under tests/golden/reference/): it widens the pinning of the oracle beyond the hand-picked cases and proves that every
 configuration the GPU sweep draws lies inside the reference's defined behaviour (so a GPU mismatch there is a bug,
 never an artefact of undefined reads)."""
 import importlib.util
@@ -20,12 +20,10 @@ _spec.loader.exec_module(gpu_fuzz)
                                           ("snes", 10), ("ntsc_conv5", 11), ("template", 12), ("pv1k", 13), ("ntsc_bloom", 14),
                                           ("pv1k", 15), ("template", 16), ("ntsc_bloom", 17)])
 def test_gpu_sweep_cases_are_inside_the_reference_domain(variant, seed):
-    if not S.have_ref(variant):
-        pytest.skip("oracle/_ref not built")
     rng = np.random.default_rng(1000 + seed)  # the same stream the GPU sweep consumes
     for case in range(4):
         fmt, outw, outh, knobs, w, h = gpu_fuzz.draw_case(rng, variant)
-        ref = S.RefEngine(variant, outw, outh, fmt, seed=1)
+        ref = S.ref_engine(variant, outw, outh, fmt, seed=1)
         ora = S.OracleEngine(variant, outw, outh, fmt)
         for e in (ref, ora):
             e.set(**knobs)
